@@ -3,6 +3,7 @@
 uniformly refined cylinder mesh, N GPUs of one node (one process per GPU).
 
   python bench.py --gpus 1 --steps K --warmup W            # this repo's CUDA path
+  python bench.py --dump-outputs bench_outputs ...          # + what the last timed step computed, as .npy (see dump_outputs)
   python bench.py --impl reference ...                      # the CPU oracle port on the host cores
   python bench.py --precond block_diagonal                  # opt-in: the CONVERGED preconditioned solve of BASELINE.json configs[1]
                                                             # (one GPU, ~80 s, its own JSON line; see run_precond)
@@ -260,6 +261,70 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_SAMPLE = 1 << 20   # global DoFs drawn for the dumped vectors: ~25 MB in all at the default size (85 M DoFs)
+DUMP_ROWS = 1 << 14     # global rows drawn for the dumped matrix entries: ~0.5 M entries of J, ~13 MB, at the default size
+
+
+def _sample(n, k, seed):
+    """All of range(n) up to k ids, else the sorted unique ids of k draws of a generator seeded with `seed`."""
+    return np.arange(n) if n <= k else np.unique(np.random.default_rng(seed).integers(0, n, k))
+
+
+def _rows_entries(rp, col, rows, l2g):
+    """Global (row, column) and CSR position of every stored entry of the local CSR rows `rows`."""
+    lens = rp[rows + 1] - rp[rows]
+    pos = np.repeat(rp[rows], lens) + np.arange(lens.sum()) - np.repeat(np.cumsum(lens) - lens, lens)
+    return np.repeat(l2g[rows], lens), l2g[col[pos]], pos
+
+
+def dump_outputs(out_dir, d, part, dev, r, its, res, rank, world, dist):
+    """--dump-outputs: write what the last timed step computed to out_dir as float64 .npy files, so that two builds can be
+    compared output for output.  Every rank takes part; rank 0 writes.
+      sample_dofs                      global DoF ids of the vector sample: _sample(n, DUMP_SAMPLE, seed 0)
+      newton_increment                 the GMRES increment (get_delta) at sample_dofs
+      residual                         the right-hand side after the Dirichlet rows (get_residual) at sample_dofs
+      jacobian_{rows,cols,values}      every stored entry of J (after the Dirichlet rows) in the global rows
+                                       _sample(n, DUMP_ROWS, seed 1), keyed by global (row, column), in that order
+      pressure_mass_{rows,cols,values} the same for the pressure mass matrix Mp (its velocity rows are empty)
+      gmres_residual_history           the residual norm after every GMRES step
+      step_scalars                     [||R||, GMRES steps, final GMRES residual]
+    The sample depends on n alone: the same ids for the same arguments."""
+    n = int(d.n)
+    dofs, rows = _sample(n, DUMP_SAMPLE, 0), _sample(n, DUMP_ROWS, 1)
+    own = part.l2g[: part.n_own]
+    picked = np.zeros(n, bool)
+    picked[dofs] = True
+    sel = np.flatnonzero(picked[own])
+    picked[:] = False
+    picked[rows] = True
+    rsel = np.flatnonzero(picked[own])
+    out = {"vectors": (own[sel], dev.get_delta()[sel], dev.get_residual()[sel])}
+    rp, col, prp, pcol = dev.get_pattern()
+    jac, pm = _rows_entries(rp, col, rsel, part.l2g), _rows_entries(prp, pcol, rsel, part.l2g)
+    del rp, col, prp, pcol          # the whole pattern and then all nnz(J) values pass through the host, one after the other
+    out["jacobian"] = jac[:2] + (dev.get_matrix_values()[jac[2]],)
+    out["pressure_mass"] = pm[:2] + (dev.get_pm_values()[pm[2]],)
+    history = dev.gmres_history()
+    if world > 1:
+        gathered = [None] * world
+        dist.all_gather_object(gathered, out)
+        out = {k: tuple(np.concatenate(a) for a in zip(*(g[k] for g in gathered))) for k in out}
+    if rank != 0:
+        return
+    g, delta, rhs = out["vectors"]
+    order = np.argsort(g)
+    assert np.array_equal(g[order], dofs)
+    files = {"sample_dofs": dofs, "newton_increment": delta[order], "residual": rhs[order],
+             "gmres_residual_history": history, "step_scalars": [r, its, res]}
+    for name in ("jacobian", "pressure_mass"):
+        i, j, v = out[name]
+        order = np.lexsort((j, i))
+        files.update({f"{name}_rows": i[order], f"{name}_cols": j[order], f"{name}_values": v[order]})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in files.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, np.float64))
+
+
 def workload_config(args, d):
     cfg = {"workload": f"synthetic uniformly refined cylinder mesh: {MESHES[args.mesh][0]} red-refined {args.levels}x, "
                        "P2-P1, state u=(sin(pi x)cos(pi y), -cos(pi x)sin(pi y)), p=xy, u_old=0.9u",
@@ -366,7 +431,13 @@ def main():
     ap.add_argument("--host-patterns", action="store_true", help="build the sparsity patterns on the host (libnst) and upload them")
     ap.add_argument("--precond", default=None, choices=["block_triangular", "block_diagonal"],
                     help="instead of the default run: the converged preconditioned solve of BASELINE.json configs[1] (one GPU, own JSON line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.precond or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the default run of the CUDA path")
     if args.precond:
         return run_precond(args)
     if args.cpu_level is None:
@@ -423,7 +494,7 @@ def main():
         if rc not in (0, -3):
             raise RuntimeError(f"nsg_solve failed: {rc}")
         ph = dev.phase_ms()
-        return r, its, ph
+        return r, its, res, ph
 
     e2e_parts = []
 
@@ -456,7 +527,7 @@ def main():
     ev0.record()
     for _ in range(args.steps):
         dev.set_delta(zero)
-        r, its, ph = step()
+        r, its, res, ph = step()
         asm_ms.append(ph["assemble"]), dir_ms.append(ph["dirichlet"]), sol_ms.append(ph["solve"])
         its_seen.append(its)
     ev1.record()
@@ -464,6 +535,8 @@ def main():
     wall_ms = 1e3 * (time.perf_counter() - t0)
     c1 = dev.counters()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:      # before the kernel timings and the extra solves below overwrite the device state
+        dump_outputs(args.dump_outputs, d, part, dev, r, its, res, rank, world, dist)
 
     # device-timed phases: max over ranks
     local_t = torch.tensor([np.mean(asm_ms) + np.mean(dir_ms), np.mean(sol_ms), wall_ms / args.steps],

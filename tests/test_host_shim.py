@@ -10,10 +10,10 @@ import pytest
 from conftest import ROOT, mesh_path
 
 HOST = os.path.join(ROOT, "navier-stokes-dealii_b200", "host")
-REF_MAIN = "/root/reference/src/main.cpp"
+# the reference's src/main.cpp (tests/golden/README.md); NS_REFERENCE_MAIN points at the original file instead
+REF_MAIN = os.environ.get("NS_REFERENCE_MAIN", mesh_path("reference_main.cpp"))
 
 
-@pytest.mark.skipif(not os.path.exists(REF_MAIN), reason="the reference tree only exists in the build container")
 def test_reference_main_compiles_and_links_unchanged(tmp_path):
     # `#include "NavierStokesSolver.hpp"` resolves next to main.cpp first, so build it from a scratch
     # directory (outside the repo) the way a maintainer would after dropping the shim header into src/
@@ -21,7 +21,7 @@ def test_reference_main_compiles_and_links_unchanged(tmp_path):
     main_cpp = tmp_path / "main.cpp"
     shutil.copyfile(REF_MAIN, main_cpp)
     exe = tmp_path / "proj"
-    cmd = ["/usr/bin/g++", "-std=c++17", "-O1", f"-I{HOST}", f"-I{ROOT}/include", str(main_cpp),
+    cmd = ["g++", "-std=c++17", "-O1", f"-I{HOST}", f"-I{ROOT}/include", str(main_cpp),
            os.path.join(HOST, "NavierStokesSolver.cpp"), f"-L{ROOT}/navier-stokes-dealii_b200", "-lnst", "-lnsg",
            f"-Wl,-rpath,{ROOT}/navier-stokes-dealii_b200", "-o", str(exe)]
     r = subprocess.run(cmd, capture_output=True, text=True)
