@@ -199,8 +199,11 @@ int nsg_time_kernel(nsg_ctx *ctx, int32_t what, int32_t reps, double *ms_per_lau
  * variants measured in round 1 (profiles/r01_summary.md) were slower and have been removed.
  * key 1 = assembly kernel variant: 0 literal 7-point quadrature loop for every term, contributions added in ascending
  * cell order as the reference's loop adds them (strict-parity kernel); 4 per-cell packets from a streaming pre-pass, one
- * (owner, cell) pair per lane, lanes sorted by commit round, first-touch stores, TMA bulk write-out (round-1 default,
- * serves any mesh); 5 (default) the "fan" scheme, see below. Variants 1-3 of round 1 were slower and have been removed.
+ * (owner, cell) pair per lane, lanes sorted by commit round, first-touch stores, TMA bulk write-out (round-1 default);
+ * 5 (default) the "fan" scheme, see below. Variants 1-3 of round 1 were slower and have been removed.
+ * Vertex valence (cells per vertex) each one serves: 5 up to 32 on oriented manifold triangulations, 4 up to 32, 0 up to
+ * 64; selecting a variant the mesh exceeds fails. A pattern built on the device (nsg_set_pattern_from_cells) holds valence
+ * up to 34 inside the domain and 33 on the boundary.
  * key 3 = Gram-Schmidt variant of SolverGMRES: 0 (default) modified, the chain of add_and_dot that deal.II
  * <= 9.4 runs (SURVEY 9-8); 1 classical (h = V^T w, w -= V h: two passes and two all-reduces per step
  * instead of k+1; deal.II >= 9.5 offers it as OrthogonalizationStrategy::classical_gram_schmidt).
@@ -218,7 +221,8 @@ int nsg_time_kernel(nsg_ctx *ctx, int32_t what, int32_t reps, double *ms_per_lau
  * key 1 = 5 (default since round 2): the "fan" scheme - one (owner, cell) pair per lane integrated in a rotated local
  * frame (owner = local vertex 0 / edge 0: all tables are immediates), the lanes of an owner in one warp in fan order,
  * shared-edge contributions combined by warp shuffles, every entry stored exactly once (no read-modify-write, no
- * commit rounds). Needs an oriented manifold triangulation; other meshes are served by 4 automatically.
+ * commit rounds). Needs an oriented manifold triangulation with valence <= 32; nsg_set_mesh serves other meshes by 4
+ * (valence <= 32) or else 0 (valence <= 64) automatically and fails on a vertex of more than 64 cells.
  * key 6 = L2 prefetch distances of variant 5 in chunks: records (low 16 bits, default 600), packets (high 16 bits, default 0). */
 int nsg_set_tuning(nsg_ctx *ctx, int32_t key, int32_t value);
 

@@ -174,6 +174,24 @@ static int upload_tables() {
 // -------------------------------------------------------------------------------------------------
 // row-owner work lists (host, once)
 // -------------------------------------------------------------------------------------------------
+// Cells per row owner (= vertex valence) each assembly variant serves: variant 0 puts an owner's pairs two per lane into
+// one warp, variant 4 one per lane (the 5-bit commit round of its record holds 0..31), the fan scheme (variant 5,
+// nsg_fanlist.inl) one per lane.
+constexpr int ASM_MAX_VALENCE_0 = 64, ASM_MAX_VALENCE_4 = 32, ASM_MAX_VALENCE_5 = 32;
+
+// the largest number of cells of one owned row owner (velocity node or pressure vertex)
+static int max_owner_cells(const nsg_ctx *c, const int32_t *cd) {
+  const int64_t nu = c->n_own_u, nown = c->n_own;
+  std::vector<int32_t> cnt((size_t)(nu / 2 + c->n_own_p), 0);
+  for (int64_t cell = 0; cell < c->n_cells; ++cell)
+    for (int k = 0; k < 9; ++k) {
+      const int32_t d = cd[15 * cell + (k < 6 ? uidx(k) : 3 * (k - 6) + 2)];
+      if (d < nu) cnt[(size_t)(d / 2)]++;
+      else if (d < nown) cnt[(size_t)(nu / 2 + d - nu)]++;
+    }
+  return cnt.empty() ? 0 : *std::max_element(cnt.begin(), cnt.end());
+}
+
 static int build_worklist(nsg_ctx *c, int kind, const int32_t *cd, WorkList *out) {
   const int64_t T = c->n_cells, nu = c->n_own_u, nown = c->n_own;
   const int64_t ng = kind == 0 ? nu / 2 : c->n_own_p;
@@ -224,7 +242,9 @@ static int build_worklist(nsg_ctx *c, int kind, const int32_t *cd, WorkList *out
       int64_t staged = 0;
       while (g < ng && g - ci.g0 < 255) {
         const int ns = nslots(g);
-        if (ns > 32) return fail(NSG_ERR_ARG, "a vertex has too many incident cells (more than 64)");
+        if (gptr[g + 1] - gptr[g] > ASM_MAX_VALENCE_0)
+          return fail(NSG_ERR_ARG, "a vertex has " + std::to_string(gptr[g + 1] - gptr[g]) + " incident cells: assembly variant 0 serves at most " +
+                                       std::to_string(ASM_MAX_VALENCE_0));
         int pos = nt;
         if ((pos & 31) + ns > 32) pos = (pos + 31) & ~31;  // next warp
         if (pos + ns > NPC) break;
@@ -392,7 +412,9 @@ static int build_worklist5(nsg_ctx *c, int kind, const int32_t *cd, WorkList *ou
       int64_t staged = 0;
       while (g < ng && g - ci.g0 < 255) {
         const int np = (int)(gptr[g + 1] - gptr[g]);
-        if (np > 31) return fail(NSG_ERR_ARG, "a vertex has too many incident cells (more than 31)");
+        if (np > ASM_MAX_VALENCE_4)
+          return fail(NSG_ERR_ARG, "a vertex has " + std::to_string(np) + " incident cells: assembly variant 4 serves at most " +
+                                       std::to_string(ASM_MAX_VALENCE_4));
         if (nt + np > NPC5 && g > ci.g0) break;
         if (g > ci.g0 && staged + stage_of(g) > stage_cap) break;
         staged += stage_of(g);
@@ -1212,7 +1234,7 @@ int nsg_set_pattern_from_cells(nsg_ctx *c, int64_t n_own_u, int64_t n_own_p, int
     NSG_CUDA(cudaMemcpyAsync(&h_err, err, 4, cudaMemcpyDeviceToHost, c->stream));
     NSG_CUDA(cudaStreamSynchronize(c->stream));
     c->d2h += 16 * (n + 1);
-    if (h_err) return fail(NSG_ERR_ARG, "a patch has more nodes than the device pattern builder holds (vertex valence > 32)");
+    if (h_err) return fail(NSG_ERR_ARG, "a patch has more nodes than the device pattern builder holds (104 velocity nodes, 40 pressure vertices: vertex valence <= 34 inside the domain, <= 33 on the boundary)");
     c->nnz = c->h_rowptr[n], c->pm_nnz = c->h_pm_rowptr[n];
     tr.mark("row lengths + scans");
     NSG_TRY(dev_alloc(&c->col, c->nnz + 16));
@@ -1313,7 +1335,14 @@ int nsg_set_mesh(nsg_ctx *c, int64_t n_cells, int64_t n_vertices, const double *
       NSG_CUDA(cudaFuncSetAttribute(k_assemble_u6<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(s6u, 1024)));
     } else {
       free_worklist(c->wl_u6), free_worklist(c->wl_p6);
-      if (c->asm_variant == 5) c->asm_variant = 4;
+      if (c->asm_variant == 5) {
+        // the fallback: variant 4 up to ASM_MAX_VALENCE_4 cells per row owner, variant 0 up to ASM_MAX_VALENCE_0
+        const int v = max_owner_cells(c, cell_dofs);
+        if (v > ASM_MAX_VALENCE_0)
+          return fail(NSG_ERR_ARG, "a vertex has " + std::to_string(v) + " incident cells: the assembly serves at most " +
+                                       std::to_string(ASM_MAX_VALENCE_0));
+        c->asm_variant = v <= ASM_MAX_VALENCE_4 ? 4 : 0;
+      }
     }
   }
   // Neumann: owned boundary P2 nodes -> (face, position on the face)
@@ -1854,7 +1883,7 @@ int nsg_set_tuning(nsg_ctx *c, int32_t key, int32_t value) {
     case 1:
       if (value != 0 && value != 4 && value != 5) return fail(NSG_ERR_ARG, "assembly variant must be 0, 4 or 5 (see nsg.h)");
       if (value == 5 && c->have_mesh && !c->fan_ok)
-        return fail(NSG_ERR_STATE, "the fan scheme (variant 5) cannot serve this mesh (not an oriented manifold triangulation)");
+        return fail(NSG_ERR_STATE, "the fan scheme (variant 5) cannot serve this mesh (not an oriented manifold triangulation with vertex valence <= 32)");
       if (value < 4) NSG_TRY(ensure_slot_worklists(c));
       if (value == 4) NSG_TRY(ensure_round_worklists(c, nullptr));
       c->asm_variant = value;

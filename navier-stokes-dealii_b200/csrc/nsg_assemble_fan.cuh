@@ -28,7 +28,9 @@
 // Summation order per entry is fixed (fan order), so the result is bitwise reproducible run to run; it differs
 // from variant 4 / the reference's cell-loop order by rounding only (1e-16 relative).
 // Meshes that are not consistently oriented, have an edge with more than two cells or a vertex with more than
-// 32 cells are detected on the host and served by variant 4.
+// 32 cells are detected on the host and served by variant 4 (up to 32 cells per vertex) or else variant 0 (up to
+// 64).  A pattern built on the device (nsg_set_pattern_from_cells) holds vertices of up to 34 cells inside the
+// domain and 33 on the boundary.
 #pragma once
 #include "nsg_assemble.cuh"
 

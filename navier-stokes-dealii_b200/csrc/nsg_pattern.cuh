@@ -97,7 +97,9 @@ __global__ void k_pat_fill(int64_t T, const int32_t *__restrict__ cell_dofs, int
   if (g >= 0) gcells[gptr[g] + atomicAdd(cursor + g, 1)] = (int32_t)cell;
 }
 
-constexpr int PAT_MAXU = 104, PAT_MAXP = 40;  // node keys of a patch: valence <= 32 gives <= 3 * 32 + 1 velocity nodes, <= 33 vertices
+// node keys of a patch: a vertex of valence v has 3 v + 1 velocity nodes and v + 1 vertices in its patch inside the domain,
+// 3 v + 3 and v + 2 on the boundary, so the builder holds valence <= 34 inside and <= 33 on the boundary
+constexpr int PAT_MAXU = 104, PAT_MAXP = 40;
 // sorted unique keys of group g: velocity nodes (key = first dof id of the node) and pressure dofs of its cells
 __device__ __forceinline__ bool pat_keys(int64_t g, const int64_t *__restrict__ gptr, const int32_t *__restrict__ gcells,
                                          const int32_t *__restrict__ cell_dofs, int32_t *ku, int &nu, int32_t *kp, int &np) {
