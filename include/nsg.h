@@ -118,7 +118,10 @@ int nsg_set_params(nsg_ctx *ctx, const nsg_params *p);
 /* assemble_system up to and including compress(add) (cpp:203-347): J = 0, R = 0, Mp = 0, the cell
  * loop with the Neumann faces, and the scatter into the fixed CSR — one call, no per-cell host
  * traffic. Reads `solution` and `solution_old` (ghosts must be current: nsg_set_solution,
- * nsg_update_solution and nsg_push_time_level keep them so). */
+ * nsg_update_solution and nsg_push_time_level keep them so). The pressure rows of J and Mp depend
+ * on the geometry and nu only: they are integrated by the first call and again only after nu,
+ * the assembly variant or a Dirichlet constraint on a pressure row changed them; R_p = 0 is
+ * written by every call. */
 int nsg_assemble(nsg_ctx *ctx);
 
 /* MatrixTools::apply_boundary_values(bv, jacobian_matrix, delta_owned, residual_vector, false)

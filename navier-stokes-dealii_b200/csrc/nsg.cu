@@ -719,17 +719,21 @@ static AsmParams asm_params(const nsg_ctx *c) {
 
 static int launch_assembly(nsg_ctx *c) {
   const AsmParams P = asm_params(c);
+  // The pressure rows of J and Mp depend on the geometry and nu only: they are integrated once and kept while
+  // c->p_rows_valid holds (see nsg_ctx).  R_p = 0 is written in every assembly, by the pressure kernel or here.
+  const bool run_p = !c->p_rows_valid;
+  if (!run_p && c->n_own_p > 0) NSG_CUDA(cudaMemsetAsync(c->R + c->n_own_u, 0, 8 * (size_t)c->n_own_p, c->stream));
   if (c->asm_variant == 5) {
-    // fan scheme.  The pressure rows depend on the geometry only: they run on a second stream beside the packet
-    // pre-pass and the velocity rows (NSG_ASM_CONCURRENT=0: one stream)
-    const bool fork = c->wl_p6.n_chunks > 0 && c->aux_stream && !(std::getenv("NSG_ASM_CONCURRENT") && std::atoi(std::getenv("NSG_ASM_CONCURRENT")) == 0);
+    // fan scheme.  The pressure rows run on a second stream beside the packet pre-pass and the velocity rows
+    // (NSG_ASM_CONCURRENT=0: one stream)
+    const bool fork = run_p && c->wl_p6.n_chunks > 0 && c->aux_stream && !(std::getenv("NSG_ASM_CONCURRENT") && std::atoi(std::getenv("NSG_ASM_CONCURRENT")) == 0);
     cudaStream_t ps = fork ? c->aux_stream : c->stream;
     if (fork) {
       NSG_CUDA(cudaEventRecord(c->ev_fork, c->stream));
       NSG_CUDA(cudaStreamWaitEvent(c->aux_stream, c->ev_fork, 0));
     }
     auto launch_p = [&]() -> int {
-      if (c->wl_p6.n_chunks > 0) {
+      if (run_p && c->wl_p6.n_chunks > 0) {
         k_assemble_p6<<<(unsigned)c->wl_p6.n_chunks, NPC6, sizeof(double) * (size_t)c->wl_p6.max_stage, ps>>>(
             c->wl_p6, c->n_own_u, c->vals, c->pm_vals, c->R, c->geom8, P);
         NSG_LAUNCH_CHECK(c);
@@ -762,16 +766,16 @@ static int launch_assembly(nsg_ctx *c) {
     else
       NSG_TRY(launch_p());
   } else if (c->asm_variant == 4) {
-    // the pressure rows depend on the geometry only: they are integrated on a second stream beside the packet
-    // pre-pass and the velocity rows (NSG_ASM_CONCURRENT=0: one stream)
-    const bool fork = c->wl_p5.n_chunks > 0 && c->aux_stream && !(std::getenv("NSG_ASM_CONCURRENT") && std::atoi(std::getenv("NSG_ASM_CONCURRENT")) == 0);
+    // the pressure rows are integrated on a second stream beside the packet pre-pass and the velocity rows
+    // (NSG_ASM_CONCURRENT=0: one stream)
+    const bool fork = run_p && c->wl_p5.n_chunks > 0 && c->aux_stream && !(std::getenv("NSG_ASM_CONCURRENT") && std::atoi(std::getenv("NSG_ASM_CONCURRENT")) == 0);
     cudaStream_t ps = fork ? c->aux_stream : c->stream;
     if (fork) {
       NSG_CUDA(cudaEventRecord(c->ev_fork, c->stream));
       NSG_CUDA(cudaStreamWaitEvent(c->aux_stream, c->ev_fork, 0));
     }
     auto launch_p = [&]() -> int {
-      if (c->wl_p5.n_chunks > 0) {
+      if (run_p && c->wl_p5.n_chunks > 0) {
         k_assemble_p5<<<(unsigned)c->wl_p5.n_chunks, NPC5, sizeof(double) * (size_t)c->wl_p5.max_stage, ps>>>(
             c->wl_p5, c->n_own_u, c->vals, c->pm_vals, c->R, c->geom, P);
         NSG_LAUNCH_CHECK(c);
@@ -811,7 +815,7 @@ static int launch_assembly(nsg_ctx *c) {
         c->wl_u, c->rowptr, c->vals, c->R, c->geom, c->cell_dofs, c->sol, c->sol_old, P);
     NSG_LAUNCH_CHECK(c);
   }
-  if (c->wl_p.n_chunks > 0) {
+  if (run_p && c->wl_p.n_chunks > 0) {
     k_assemble_p<<<(unsigned)c->wl_p.n_chunks, NPC, sizeof(double) * (size_t)c->wl_p.max_stage, c->stream>>>(
         c->wl_p, c->n_own_u, c->rowptr, c->vals, c->pm_rowptr, c->pm_vals, c->R, c->geom, P);
     NSG_LAUNCH_CHECK(c);
@@ -823,6 +827,7 @@ static int launch_assembly(nsg_ctx *c) {
                                                                         c->cell_vertices, c->xy, c->R, P);
     NSG_LAUNCH_CHECK(c);
   }
+  c->p_rows_valid = true;
   return NSG_OK;
 }
 
@@ -1541,6 +1546,7 @@ int nsg_set_params(nsg_ctx *c, const nsg_params *p) {
   if (!c || !p) return fail(NSG_ERR_ARG, "null argument");
   if (!(p->nu > 0) || (p->use_mass && !(p->deltat > 0))) return fail(NSG_ERR_ARG, "nu and deltat must be positive");
   if (p->dirichlet_diag < 0 || p->dirichlet_diag > 1) return fail(NSG_ERR_ARG, "dirichlet_diag must be 0 (Trilinos rule) or 1 (keep a non-zero diagonal)");
+  if (p->nu != c->prm.nu) c->p_rows_valid = false;  // the only parameter the pressure-row kernels read (Mp = table/nu)
   c->prm = *p;
   return NSG_OK;
 }
@@ -1593,6 +1599,7 @@ int nsg_apply_dirichlet(nsg_ctx *c, int64_t n, const int32_t *dofs, const double
   // have constrained rows (the per-block apply_boundary_values returns early otherwise)
   bool has_blk[2] = {false, false};
   for (int64_t i = 0; i < n && !(has_blk[0] && has_blk[1]); ++i) has_blk[dofs[i] < c->n_own_u ? 0 : 1] = true;
+  if (has_blk[1]) c->p_rows_valid = false;  // a constrained pressure row: the next assembly integrates the pressure rows again
   NSG_CUDA(cudaMemsetAsync(c->first_idx, 0xff, 16, c->stream));
   for (int b = 0; b < 2; ++b) {
     if (!has_blk[b]) continue;
@@ -1886,6 +1893,7 @@ int nsg_set_tuning(nsg_ctx *c, int32_t key, int32_t value) {
         return fail(NSG_ERR_STATE, "the fan scheme (variant 5) cannot serve this mesh (not an oriented manifold triangulation with vertex valence <= 32)");
       if (value < 4) NSG_TRY(ensure_slot_worklists(c));
       if (value == 4) NSG_TRY(ensure_round_worklists(c, nullptr));
+      if (value != c->asm_variant) c->p_rows_valid = false;
       c->asm_variant = value;
       return NSG_OK;
     default: return fail(NSG_ERR_ARG, "unknown tuning key");

@@ -520,6 +520,8 @@ k_assemble_u6(const WorkList wl, double *__restrict__ vals, double *__restrict__
 // Record as above; off[0..5] = column pairs of the rotated P2 nodes in the Jacobian row, off[6..8] = the three
 // pressure columns in the pressure-mass row, off[9] = image offset of the Jacobian row, off[10] = offset of the
 // pressure-mass row in the mass image.  The p-p block of the Jacobian is never written: the image is zero-filled.
+// Reads the geometry and nu only, so launch_assembly runs it once and again only after nu, the assembly variant or a
+// Dirichlet constraint on a pressure row changed what it writes (nsg_ctx::p_rows_valid).
 __global__ void __launch_bounds__(NPC6, (6 * 128) / NPC6)
 k_assemble_p6(const WorkList wl, int64_t n_own_u, double *__restrict__ vals, double *__restrict__ pm_vals, double *__restrict__ R,
               const double *__restrict__ geom8, const AsmParams P) {

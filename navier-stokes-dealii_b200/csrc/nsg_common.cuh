@@ -228,6 +228,12 @@ struct nsg_ctx {
   nsg::WorkList wl_u6, wl_p6;  // assembly variant 5 ("fan"): the lanes of an owner in one warp, every entry stored once
   int asm_pf_rec = 600, asm_pf_pk = 0;  // variant 5: L2 prefetch distances in chunks (tuning key 6; measured: records 600 ahead -3 %)
   bool fan_ok = false;         // the mesh is an oriented manifold triangulation the fan scheme can serve
+  // The pressure rows of J (B and the zero p-p block) and all of Mp hold what the pressure-row kernel of asm_variant
+  // computes from the geometry and nu: launch_assembly skips that kernel while this is set.  Cleared by nsg_set_params
+  // when nu changes, by nsg_apply_dirichlet when it constrains a pressure row and by nsg_set_tuning when the assembly
+  // variant changes (the variants sum in different orders).  Pattern and mesh are set once, before the first assembly.
+  // Per context: with several ranks each context holds only its owned pressure rows.
+  bool p_rows_valid = false;
   // Neumann: boundary nodes -> faces
   int64_t n_bnodes = 0;
   int32_t *bnode_dof = nullptr, *bnode_ptr = nullptr, *bnode_face = nullptr, *bnode_pos = nullptr;
