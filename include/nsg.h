@@ -171,12 +171,36 @@ int nsg_get_delta(nsg_ctx *ctx, double *host);
 int nsg_get_residual(nsg_ctx *ctx, double *host);
 int nsg_get_matrix_values(nsg_ctx *ctx, double *host /* nnz(J), CSR order */);
 int nsg_get_pm_values(nsg_ctx *ctx, double *host /* nnz(Mp) */);
+/* The counterpart of nsg_get_solution_ghosted: writes the owned entries AND the ghost layer of `solution` as given (n_loc
+ * doubles), with no exchange. Lets one GPU hold the P per-rank contexts of a partition with correct ghost values. */
+int nsg_set_solution_ghosted(nsg_ctx *ctx, const double *host);
 
 /* N3 (SURVEY 8f; the reference has no drag/lift code): force of the fluid on the body bounded by the
  * faces with `boundary_id` (13 = cylinder, cpp:368), from the current `solution`:
  * F = -oint (rho nu grad(u) n - p n) ds, n = outward normal of the fluid domain, integrated with the
  * reference's 3-point face rule (cpp:52). out2 = (drag F_x, lift F_y), global over all ranks. */
 int nsg_boundary_force(nsg_ctx *ctx, int32_t boundary_id, double *out2);
+
+/* Global cell ids (nst_part_cell_ids) and ownership flags (nst_part_cell_owned) of the n_cells local cells, for
+ * nsg_eval_points. Call after nsg_set_mesh. Without it every local cell is owned and its global id is its local index,
+ * which is right for P = 1. */
+int nsg_set_cell_ownership(nsg_ctx *ctx, const int32_t *global_cell_id, const uint8_t *owned);
+
+/* Point evaluation of the current `solution` (probes, the pressure difference across a body, transfer to another mesh):
+ * locates the n points xy[2n] in the mesh and evaluates there u_x, u_y, p (values[3n], point-major) and, if grads is not
+ * NULL, du_x/dx, du_x/dy, du_y/dx, du_y/dy, dp/dx, dp/dy (grads[6n]); cell[n] (may be NULL) gets the global id of the
+ * cell used. A point lies in a cell when its three barycentric coordinates are >= -1e-12; of the owned cells containing
+ * it the one with the smallest global id is used, so the result does not depend on the rank count. A point no cell
+ * contains (or with a non-finite coordinate) gets cell -1 and NaN values. The spatial index (a uniform grid of bins) is
+ * built on the first call. collective != 0 on a context with a communicator: every rank passes the same points and
+ * receives the same results (NCCL all-reduce of the winning cell id, then of the values); otherwise each context
+ * answers from its own owned cells. n = 0 does nothing; before nsg_set_mesh: NSG_ERR_STATE. */
+int nsg_eval_points(nsg_ctx *ctx, int64_t n, const double *xy, int32_t collective, double *values, double *grads,
+                    int64_t *cell);
+/* The spatial index of nsg_eval_points (NSG_ERR_STATE before the first call): out8 = bins in x, bins in y, bin side,
+ * cell entries, non-empty bins, entries of the largest bin, index bytes (8 (bins + 1) + 4 entries), build time in ms
+ * (host clock, ending in a device synchronise). */
+int nsg_points_index_info(nsg_ctx *ctx, double *out8);
 
 /* Building blocks exported for parity tests and roofline measurement. x, y are host vectors of
  * owned length. nsg_spmv: y = J x (jacobian_matrix.vmult). nsg_precond_apply: y = P^-1 x for the
@@ -191,7 +215,8 @@ int nsg_ilu_apply(nsg_ctx *ctx, int32_t which, const double *x, double *y);
  * Neumann, no Dirichlet), 1 = SpMV J*delta, 2 = add_and_dot, 3 = dot, 4 = one halo exchange, 5 = FP64 pipe
  * micro-benchmark (SM count x 16 CTAs x 256 threads x 8 chains x 2048 dependent DFMA = SMs x 67 108 864 DFMA per launch,
  * 2 flop each: the measured FP64 peak the assembly's FP64-pipe share is quoted against), 6 / 7 = one ILU(0) apply (forward +
- * backward triangular solve, tuning key 4) of the velocity / pressure-mass block, factorised before the timed region. */
+ * backward triangular solve, tuning key 4) of the velocity / pressure-mass block, factorised before the timed region,
+ * 8 = locate + evaluate the points of the last nsg_eval_points call (local mode, without the host copies). */
 int nsg_time_kernel(nsg_ctx *ctx, int32_t what, int32_t reps, double *ms_per_launch);
 
 /* Tuning knobs that do not change what is computed (only the summation order inside a row):

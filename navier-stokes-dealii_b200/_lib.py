@@ -154,7 +154,11 @@ _NSG_SIGS = {
     "nsg_get_residual": (C.c_int, [vp, f64p]),
     "nsg_get_matrix_values": (C.c_int, [vp, f64p]),
     "nsg_get_pm_values": (C.c_int, [vp, f64p]),
+    "nsg_set_solution_ghosted": (C.c_int, [vp, f64p]),
     "nsg_boundary_force": (C.c_int, [vp, i32, f64p]),
+    "nsg_set_cell_ownership": (C.c_int, [vp, i32p, u8p]),
+    "nsg_eval_points": (C.c_int, [vp, i64, f64p, i32, f64p, _opt(f64p), _opt(i64p)]),
+    "nsg_points_index_info": (C.c_int, [vp, f64p]),
     "nsg_spmv": (C.c_int, [vp, f64p, f64p]),
     "nsg_precond_apply": (C.c_int, [vp, i32, f64p, f64p]),
     "nsg_ilu_apply": (C.c_int, [vp, i32, f64p, f64p]),

@@ -939,6 +939,7 @@ static int get_vec(nsg_ctx *c, const double *dev, double *host, int64_t n) {
 #include "nsg_krylov.cuh"
 #include "nsg_precond.cuh"
 #include "nsg_gmres_fused.cuh"
+#include "nsg_points.cuh"
 
 
 namespace nsg {
@@ -1074,6 +1075,7 @@ void nsg_destroy(nsg_ctx *c) {
   free_worklist(c->wl_u), free_worklist(c->wl_p), free_worklist(c->wl_u5), free_worklist(c->wl_p5);
   free_worklist(c->wl_u6), free_worklist(c->wl_p6);
   dev_free(c->geom8);
+  pt_free(c);
   dev_free(c->bnode_dof), dev_free(c->bnode_ptr), dev_free(c->bnode_face), dev_free(c->bnode_pos);
   dev_free(c->bface_cell), dev_free(c->bface_face), dev_free(c->bface_tag);
   dev_free(c->sol), dev_free(c->sol_old), dev_free(c->delta), dev_free(c->R), dev_free(c->basis), dev_free(c->work);
@@ -1757,6 +1759,12 @@ int nsg_get_delta(nsg_ctx *c, double *h) { return get_owned(c, c ? c->delta : nu
 int nsg_get_residual(nsg_ctx *c, double *h) { return get_owned(c, c ? c->R : nullptr, h, c ? c->n_own : 0); }
 int nsg_get_matrix_values(nsg_ctx *c, double *h) { return get_owned(c, c ? c->vals : nullptr, h, c ? c->nnz : 0); }
 int nsg_get_pm_values(nsg_ctx *c, double *h) { return get_owned(c, c ? c->pm_vals : nullptr, h, c ? c->pm_nnz : 0); }
+int nsg_set_solution_ghosted(nsg_ctx *c, const double *h) {
+  if (!c || !h) return fail(NSG_ERR_ARG, "null argument");
+  if (!c->have_pattern) return fail(NSG_ERR_STATE, "nsg_set_pattern first");
+  NSG_CUDA(cudaSetDevice(c->device));
+  return put_vec(c, c->sol, h, c->n_loc);
+}
 
 int nsg_spmv(nsg_ctx *c, const double *x, double *y) {
   if (!c || !x || !y) return fail(NSG_ERR_ARG, "null argument");
@@ -1818,6 +1826,50 @@ int nsg_boundary_force(nsg_ctx *c, int32_t boundary_id, double *out2) {
   return NSG_OK;
 }
 
+int nsg_set_cell_ownership(nsg_ctx *c, const int32_t *global_cell_id, const uint8_t *owned) {
+  if (!c || !global_cell_id || !owned) return fail(NSG_ERR_ARG, "null argument");
+  if (!c->have_mesh) return fail(NSG_ERR_STATE, "nsg_set_mesh first");
+  for (int64_t i = 0; i < c->n_cells; ++i)
+    if (global_cell_id[i] < 0 || global_cell_id[i] == PT_NONE) return fail(NSG_ERR_ARG, "global cell id out of range");
+  NSG_CUDA(cudaSetDevice(c->device));
+  dev_free(c->cell_gid), dev_free(c->cell_owned);
+  NSG_TRY(upload(c, &c->cell_gid, global_cell_id, c->n_cells));
+  NSG_TRY(upload(c, &c->cell_owned, owned, c->n_cells));
+  NSG_CUDA(cudaStreamSynchronize(c->stream));
+  return NSG_OK;
+}
+
+int nsg_eval_points(nsg_ctx *c, int64_t n, const double *xy, int32_t collective, double *values, double *grads, int64_t *cell) {
+  if (!c || n < 0) return fail(NSG_ERR_ARG, "bad argument");
+  if (!c->have_mesh) return fail(NSG_ERR_STATE, "nsg_set_mesh first");
+  if (n == 0) return NSG_OK;
+  if (!xy || !values) return fail(NSG_ERR_ARG, "null argument");
+  NSG_CUDA(cudaSetDevice(c->device));
+  if (!c->pidx.built) NSG_TRY(pt_build_index(c));
+  NSG_TRY(pt_ensure_scratch(c, n, grads != nullptr));
+  PointIndex &P = c->pidx;
+  NSG_CUDA(cudaMemcpyAsync(P.pxy, xy, 16 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
+  NSG_TRY(pt_run(c, n, collective && c->n_ranks > 1 && c->comm, grads != nullptr));
+  NSG_CUDA(cudaMemcpyAsync(values, P.vals, 24 * (size_t)n, cudaMemcpyDeviceToHost, c->stream));
+  if (grads) NSG_CUDA(cudaMemcpyAsync(grads, P.grads, 48 * (size_t)n, cudaMemcpyDeviceToHost, c->stream));
+  if (cell) NSG_CUDA(cudaMemcpyAsync(cell, P.cell, 8 * (size_t)n, cudaMemcpyDeviceToHost, c->stream));
+  NSG_CUDA(cudaStreamSynchronize(c->stream));
+  P.last_n = n, P.last_grads = grads != nullptr;
+  c->h2d += 16 * n;
+  c->d2h += (24 + (grads ? 48 : 0) + (cell ? 8 : 0)) * n;
+  return NSG_OK;
+}
+
+int nsg_points_index_info(nsg_ctx *c, double *out8) {
+  if (!c || !out8) return fail(NSG_ERR_ARG, "null argument");
+  const PointIndex &P = c->pidx;
+  if (!P.built) return fail(NSG_ERR_STATE, "no point index yet: it is built by the first nsg_eval_points");
+  const int64_t nb = (int64_t)P.grid.nx * P.grid.ny;
+  out8[0] = P.grid.nx, out8[1] = P.grid.ny, out8[2] = P.h, out8[3] = (double)P.n_entries;
+  out8[4] = (double)P.n_nonempty, out8[5] = P.max_bin, out8[6] = 8.0 * (nb + 1) + 4.0 * P.n_entries, out8[7] = P.build_ms;
+  return NSG_OK;
+}
+
 int nsg_time_kernel(nsg_ctx *c, int32_t what, int32_t reps, double *ms_per_launch) {
   if (!c || !ms_per_launch || reps < 1) return fail(NSG_ERR_ARG, "bad argument");
   if (!c->have_mesh) return fail(NSG_ERR_STATE, "nsg_set_mesh first");
@@ -1826,9 +1878,11 @@ int nsg_time_kernel(nsg_ctx *c, int32_t what, int32_t reps, double *ms_per_launc
   double *a = c->work + 2 * c->stride, *b = c->work + 3 * c->stride, *w = c->work + 4 * c->stride;
   NSG_CUDA(cudaMemsetAsync(c->scal, 0, 8, c->stream));
   if (what == 6 || what == 7) NSG_TRY(precond_initialize(c));  // factorise outside the timed region
+  if (what == 8 && c->pidx.last_n == 0) return fail(NSG_ERR_STATE, "kernel 8 repeats the last nsg_eval_points: none yet");
   NSG_CUDA(cudaEventRecord(c->ev0, c->stream));
   for (int r = 0; r < reps; ++r) {
     switch (what) {
+      case 8: NSG_TRY(pt_run(c, c->pidx.last_n, false, c->pidx.last_grads)); break;  // locate + evaluate, local mode
       case 6: NSG_TRY(ilu_apply(c, c->blkA, b, a)); break;            // ILU(0) apply of the velocity block (tuning key 4)
       case 7: NSG_TRY(ilu_apply(c, c->blkM, b + c->n_own_u, a + c->n_own_u)); break;  // ... of the pressure mass block
       case 0: NSG_TRY(launch_assembly(c)); break;

@@ -183,6 +183,27 @@ struct CsrBlock {  // a sub-matrix held separately (A, Mp, B of the block precon
   bool tri_pick = false;        // ... and the one-CTA solve is estimated faster than the stamped single launch
 };
 
+// Point location (nsg_points.cuh): the uniform bin grid over the cells, built on the first nsg_eval_points, and the
+// per-point scratch of the last call (grown on demand).
+struct PtGrid {
+  double x0, y0, inv_h;  // bin of x: floor((x - x0) * inv_h)
+  int32_t nx, ny;
+};
+struct PointIndex {
+  bool built = false;
+  PtGrid grid{};
+  double h = 0, build_ms = 0;
+  int64_t n_entries = 0, n_nonempty = 0;
+  int32_t max_bin = 0;
+  int64_t *start = nullptr;    // [nx*ny+1] first entry of each bin
+  int32_t *entries = nullptr;  // [n_entries] local cell ids
+  int64_t cap = 0, grads_cap = 0, last_n = 0;
+  bool last_grads = false;
+  double *pxy = nullptr, *vals = nullptr, *grads = nullptr;  // [2n], [3n], [6n]
+  int32_t *gid = nullptr, *win = nullptr, *loc = nullptr;   // located global id, winning global id, located local cell
+  int64_t *cell = nullptr;                                   // [n] result cell id (-1: not found)
+};
+
 }  // namespace nsg
 
 struct nsg_ctx {
@@ -293,4 +314,8 @@ struct nsg_ctx {
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaStream_t aux_stream = nullptr;  // pressure-row assembly runs beside the velocity rows
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+  // point evaluation: global cell ids and ownership (nsg_set_cell_ownership; nullptr = local index, all owned) and the index
+  int32_t *cell_gid = nullptr;
+  uint8_t *cell_owned = nullptr;
+  nsg::PointIndex pidx;
 };

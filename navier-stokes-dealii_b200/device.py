@@ -45,6 +45,7 @@ class DeviceProblem:
 
     def comm_init(self, rank, n_ranks, unique_id):
         nsg_check(self._L.nsg_comm_init(self._h, int(rank), int(n_ranks), C.create_string_buffer(unique_id, 128)))
+        self._comm = True
         p = self.part
         nsg_check(self._L.nsg_set_halo(self._h, p.n_neighbors, _nz(p.neighbors), p.send_ptr, _nz(p.send_idx), p.recv_ptr,
                                        _nz(p.recv_idx)))
@@ -190,11 +191,46 @@ class DeviceProblem:
     def get_pm_values(self):
         return self._get(self._L.nsg_get_pm_values, self.pm_nnz)
 
+    def set_solution_ghosted(self, v):
+        """Owned entries followed by the ghost layer, written as given (no exchange): the inverse of get_solution_ghosted."""
+        v = np.ascontiguousarray(v, np.float64)
+        if v.shape != (self.part.n_loc,):
+            raise ValueError(f"expected {self.part.n_loc} owned + ghost entries, got {v.shape}")
+        nsg_check(self._L.nsg_set_solution_ghosted(self._h, v))
+
     def boundary_force(self, boundary_id):
         """(drag, lift) on the body bounded by the faces with this boundary id (N3)."""
         out = np.zeros(2)
         nsg_check(self._L.nsg_boundary_force(self._h, int(boundary_id), out))
         return out
+
+    def evaluate(self, points, gradients=False, collective=None):
+        """u_x, u_y, p of the current solution at points (n, 2): returns values (n, 3), then grads (n, 2, 3) with
+        grads[i, d, k] = d(value k)/dx_d if gradients, then cells (n,), the global id of the cell used (-1 and NaN values
+        where no cell contains the point). collective=None: collective exactly when comm_init was called; then every rank
+        passes the same points and gets the same results."""
+        pts = np.ascontiguousarray(points, np.float64)
+        if pts.ndim != 2 or pts.shape[1] != 2:
+            raise ValueError(f"points must have shape (n, 2), got {pts.shape}")
+        if not getattr(self, "_ownership_set", False):   # first use: global cell ids and ownership of the partition
+            nsg_check(self._L.nsg_set_cell_ownership(self._h, _nz(self.part.cell_ids), _nz(self.part.cell_owned, np.uint8)))
+            self._ownership_set = True
+        if collective is None:
+            collective = getattr(self, "_comm", False)
+        n = len(pts)
+        vals = np.empty((max(n, 1), 3), np.float64)
+        grads = np.empty((max(n, 1), 3, 2), np.float64) if gradients else None
+        cells = np.empty(max(n, 1), np.int64)
+        nsg_check(self._L.nsg_eval_points(self._h, n, _nz(pts.reshape(-1), np.float64), 1 if collective else 0, vals.reshape(-1),
+                                          None if grads is None else grads.reshape(-1), cells))
+        return (vals[:n],) + ((grads[:n].transpose(0, 2, 1),) if gradients else ()) + (cells[:n],)
+
+    def points_index_info(self):
+        """The spatial index of evaluate() (built by its first call)."""
+        o = np.zeros(8)
+        nsg_check(self._L.nsg_points_index_info(self._h, o))
+        return {"bins_x": int(o[0]), "bins_y": int(o[1]), "bin_side": o[2], "entries": int(o[3]), "nonempty_bins": int(o[4]),
+                "max_bin": int(o[5]), "bytes": int(o[6]), "build_ms": o[7]}
 
     def spmv(self, x):
         x = np.ascontiguousarray(x, np.float64)

@@ -61,6 +61,7 @@ class Parameters:
     output_dir: str = ""                             # "" = no files (cpp:681-728 writes XDMF/HDF5)
     dirichlet_diag: int = 0                          # include/nsg.h nsg_params: 0 TrilinosWrappers rule, 1 keep a non-zero diagonal
     force_boundary_id: int = -1                      # >= 0: record drag/lift on this boundary after every time step (N3)
+    probe_points: tuple = ()                         # (x, y) points: record (u_x, u_y, p) there after every time step
     extra: dict = field(default_factory=dict)
 
 
@@ -92,6 +93,7 @@ class NavierStokesSolver:
         self.time = 0.0
         self.history = []        # (time_step, newton_iter, residual_norm, gmres_its)
         self.force_history = []  # (time, F_x, F_y) when Parameters.force_boundary_id >= 0
+        self.probe_history = []  # (time, values (n, 3)) when Parameters.probe_points is not empty
 
     def pcout(self, *a, **k):
         if self.verbose:
@@ -238,6 +240,8 @@ class NavierStokesSolver:
             if self.prm.force_boundary_id >= 0:
                 f = self.dev.boundary_force(self.prm.force_boundary_id)
                 self.force_history.append((self.time, float(f[0]), float(f[1])))
+            if len(self.prm.probe_points):
+                self.probe_history.append((self.time, self.point_values(self.prm.probe_points)))
             self.output(time_step, self.time)
             self.pcout("")
 
@@ -266,6 +270,32 @@ class NavierStokesSolver:
         """Force (F_x, F_y) and the coefficients 2F/(rho U^2 D)."""
         f = self.dev.boundary_force(boundary_id)
         return f, 2.0 * f / (self.prm.rho * u_mean ** 2 * diameter)
+
+    # ---- point evaluation: probes, the pressure difference across the cylinder, transfer to another mesh ---------------
+    def point_values(self, points):
+        """(u_x, u_y, p) of the current solution at points (n, 2); NaN where no cell contains a point. With P > 1 every
+        rank must pass the same points and gets the same values."""
+        return self.dev.evaluate(np.asarray(points, np.float64).reshape(-1, 2))[0]
+
+    def pressure_difference(self, front=(-0.5, 0.0), back=(0.5, 0.0)):
+        """p(front) - p(back): the DFG cylinder benchmark's delta p (the repository's meshes: cylinder of radius 0.5 at
+        the origin)."""
+        v = self.point_values([front, back])
+        return float(v[0, 2] - v[1, 2])
+
+    def set_solution_from(self, source):
+        """Interpolate the solution of another solver (e.g. on a coarser mesh of the same domain) at this solver's support
+        points and make it the current solution (deal.II's VectorTools::interpolate_to_different_mesh). P = 1 only."""
+        if self.world_size > 1 or source.world_size > 1:
+            raise NotImplementedError("set_solution_from: transfer between partitioned meshes is not implemented")
+        own = np.asarray(self.part.l2g[: self.part.n_own])
+        xy = self.dofs.support_points()[own]
+        vals, cells = source.dev.evaluate(xy)
+        if (cells < 0).any():
+            bad = np.flatnonzero(cells < 0)
+            raise ValueError(f"{len(bad)} support points lie outside the source mesh (first at {xy[bad[0]].tolist()})")
+        comp = np.where(own < self.dofs.n_u, own % 2, 2)
+        self.dev.set_solution(vals[np.arange(len(own)), comp])
 
     # ---- helpers ----------------------------------------------------------------------------------
     def gather_solution(self):
